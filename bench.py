@@ -42,18 +42,27 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 ITERS = 10
 N_FRAMES = 20
 KTIME_EVERY = 5
 SHARD_BLOCK_M = 64
 METRIC = "scans/sec (24k-pt sweep vs 1M-pt map); kNN+Jacobian HBM GB/s vs peak"
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=positive_int, default=200, help="timed steps (scans) of every timed leg")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--multi", default="sharded", choices=["sharded", "replicas"])
@@ -68,7 +77,36 @@ def parse():
     ap.add_argument("--workload", default="", choices=["", "horizon", "rot", "stream"],
                     help="horizon: configs[1] (default at N = 1); rot: configs[2]; stream: configs[4]'s streamed workload "
                          "(130k sweep, 10 M-pt map as 20 frames, map maintenance in the step; default at N > 1, also runs at N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last timed step returned to its caller as DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB in all), so that two builds can be compared output for output")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: array} as out_dir/<name>.npy.  Point clouds (records of float32 fields) become [n, fields] float32,
+    float32 stays float32, everything else becomes float64.  If the whole set exceeds DUMP_BUDGET_BYTES, every cloud keeps
+    the same fraction of its rows, chosen by a fixed seed (the same rows for the same shapes, run after run)."""
+    out = {}
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a)
+        if a.dtype.fields is not None:
+            a = a.view(np.float32).reshape(len(a), -1)
+        elif a.dtype != np.float32:
+            a = a.astype(np.float64)
+        out[name] = a
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_BUDGET_BYTES:
+        clouds = [name for name, a in out.items() if a.ndim > 1]
+        small = total - sum(out[name].nbytes for name in clouds)
+        keep = (DUMP_BUDGET_BYTES - small) / (total - small)
+        for name in clouds:
+            a = out[name]
+            rows = np.random.default_rng(0).choice(len(a), int(len(a) * keep), replace=False)
+            out[name] = a[np.sort(rows)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peak():
@@ -354,13 +392,15 @@ def run_reference(args):
         probe[nt] = float(np.median(ts))
     best_nt = min(probe, key=probe.get)
     warm = max(args.warmup, 3) if not heavy else 1
-    steps = max(1, min(args.steps, int(45.0 / max(probe[best_nt], 1e-3))))
+    steps = args.steps
     for k in range(warm):
         W.scan(k, best_nt)
     t0 = time.perf_counter()
     for k in range(steps):
-        W.scan(k, best_nt)
+        last = W.scan(k, best_nt)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pose": last[0], "queries": [last[1]]})
     val = steps / dt
     sample = (f"{steps} scans (extract + VoxelGrid + {ITERS} GN iters" + (", + map maintenance: VoxelGrid of the 20-frame concatenation and kd-tree build per scan" if heavy else
               f", kd-tree prebuilt in {W.t_setup:.2f}s, excluded — the reference rebuilds it per scan, L/src/LidarOdometry.cpp:490") + ")")
@@ -611,7 +651,7 @@ def bench_body(args, fallback_note=None):
             d2h = (len(surf) + len(edge) + len(cut)) * psz + len(ds) * psz + 56
             if stream_wl:
                 h2d += push_host()
-            return pose, h2d, d2h
+            return pose, h2d, d2h, (surf, edge, cut, ds)
 
         def push_host():
             """buildLocalMap's push with the frame arriving from the host, then the rebuild; returns the bytes uploaded."""
@@ -723,6 +763,7 @@ def bench_body(args, fallback_note=None):
             for v in cx_phase_ms.values():
                 v[:] = [0.0, 0.0, 0.0, 0.0, 0]
         ms_res_local, last = timed(step_resident, steps, warmup, prep_for(ctx), after_warmup=after_warm)
+        outputs = {"pose": np.array(last[0]), "queries": [last[1]]}
         phases_main = list(cx_phase_ms.get(id(ctx), [0, 0, 0, 0, 0]))
         cnt = ctx.counters(reset=True)
         # C-bar of the LAST timed scan's queries at its start pose, while they are still resident (the later legs replace them)
@@ -730,6 +771,10 @@ def bench_body(args, fallback_note=None):
         ms_res, ms_res_ranks = over_ranks(ms_res_local)
         # ---- timed region 2: end to end with host buffers
         ms_seq_local, last_seq = timed(step_e2e, steps, warmup)
+        if args.dump_outputs:        # copies: the two-node leg below reuses the pose and down-sampled-cloud buffers
+            outputs["e2e_pose"] = np.array(last_seq[0])
+            for name, cloud in zip(("surf", "edge", "cut", "surf_ds"), last_seq[3]):
+                outputs["e2e_" + name] = np.array(cloud)
         ms_seq, _ = over_ranks(ms_seq_local)
         # Sharded runs keep the one-thread e2e leg.  The two-node leg put each rank's GN exchange (a kernel that waits for its
         # peers) next to a second host thread and context on the same GPU; it ran on 2 GPUs, but on 8 every rank's exchange
@@ -972,6 +1017,8 @@ def bench_body(args, fallback_note=None):
             line["speedup_vs_1gpu_same_workload"] = value / same1["value"]
     if fallback_note or exchange_note:
         line["note"] = "; ".join(x for x in (fallback_note, exchange_note) if x)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     ctx.close()
     return None

@@ -124,6 +124,30 @@ def test_clock_sampler_keeps_the_rows_inside_the_window(tmp_path, monkeypatch):
     assert off.summary()["samples"] == 0 and off.summary()["sm_mhz"] is None
 
 
+def test_dump_outputs_types_and_budget(tmp_path, monkeypatch):
+    """--dump-outputs: clouds become [n, fields] float32 with their bits kept, the pose stays float64, counts become float64;
+    over the size budget every cloud keeps the same seeded sample of rows, identical from run to run, and the pose stays whole."""
+    import numpy as np
+    import bench
+    from liliom_b200 import PT48
+    cloud = np.zeros(1000, PT48)
+    cloud["x"] = np.arange(1000, dtype=np.float32); cloud["curvature"] = 0.1
+    pose = np.array([1.0, 0, 0, 0, 0.1, 0.2, 0.3])
+    bench.dump_outputs(str(tmp_path / "a"), {"surf": cloud, "pose": pose, "queries": [1409]})
+    s = np.load(tmp_path / "a" / "surf.npy")
+    assert s.dtype == np.float32 and s.shape == (1000, 12) and s.tobytes() == cloud.tobytes()
+    p = np.load(tmp_path / "a" / "pose.npy")
+    assert p.dtype == np.float64 and p.tobytes() == pose.tobytes()
+    assert np.load(tmp_path / "a" / "queries.npy").tolist() == [1409.0]
+    monkeypatch.setattr(bench, "DUMP_BUDGET_BYTES", 12_000)
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), {"surf": cloud, "pose": pose})
+    b, c = np.load(tmp_path / "b" / "surf.npy"), np.load(tmp_path / "c" / "surf.npy")
+    assert sum(np.load(tmp_path / "b" / f).nbytes for f in ("surf.npy", "pose.npy")) <= 12_000
+    assert 0 < len(b) < 1000 and np.array_equal(b, c) and np.all(np.diff(b[:, 0]) > 0)
+    assert np.load(tmp_path / "b" / "pose.npy").tobytes() == pose.tobytes()
+
+
 def test_two_node_leg_is_fail_safe():
     """bench.resolve_e2e: the optional two-node e2e leg may fail on any rank; then EVERY rank reports the one-thread figure (decided on
     the gathered per-rank times, so the ranks' collectives stay matched) and the line says so."""
